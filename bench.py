@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — benchmarks of the B200 DirectXTex backend on the BASELINE.json configurations.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5] [--impl reference] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c2|c3|c4|c5] [--impl reference] [--batch B] [--dump-outputs DIR]
 
 Default (= the headline, BASELINE.json `metric`, configs[1]):  Mtexels/s BC7 encode, 4096x4096 RGBA32F -> BC7_UNORM,
 TEX_COMPRESS_DEFAULT.  A step = one pass of the hot path over a batch of B (default 32) 4096^2 images per GPU, so that the
@@ -17,7 +17,11 @@ Prints ONE JSON line (rank 0):  `value` = device-resident throughput (inputs in 
 host-pointer C ABI with pinned host buffers (H2D + D2H inside the timed region), `roofline` = the dominant kernel against the
 measured HBM peak, `cpu_baseline` = the UNMODIFIED reference (oracle/_ref) on the host cores on a bounded sample, `parity` =
 the result of this very run checked against the reference (SURVEY 8(d): parity checks run with every measurement).
-`--impl reference` times the reference's own CPU implementation on a bounded sample per step.
+`--impl reference` times the reference's own CPU implementation on a bounded sample per step.  `cpu_baseline` and `parity` are
+null where the reference build (oracle/Makefile) is absent.
+`--dump-outputs DIR` writes what the last timed step computed (rank 0), as DIR/<name>.npy in float32: every output buffer of
+the step, or a fixed seeded sample of its 16-byte rows where the outputs together exceed 60 MiB.  The inputs are seeded, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes as C
@@ -180,6 +184,9 @@ class C2:
             raise ctx.capi.DxTexError(hr, "dxb200_compress_device")
         return e0, e1, self.d_out[i & 1]
 
+    def outputs(self, ctx):
+        return {"bc7_blocks": self.d_out[ctx.last_step & 1]}
+
     def alternates(self, ctx):
         """the same batch through the other feed of the BC7 kernel (dxb200_set_option(DXB200_OPT_BC7_FEED, ..)): ms per step, output equal.
         The default (4 = automatic) feeds batches by TMA tensor-map tile loads (k_compress_bc7_tma) and single images by direct loads."""
@@ -322,6 +329,9 @@ class C3:
         ctx.extra_events.setdefault("mips_cubic", []).append((m0, m1))
         return e0, e1, self.d_out[i & 1]
 
+    def outputs(self, ctx):
+        return {"mip_chain_rgba16f": self.d_chain.view(ctx.torch.float16), "bc6h_blocks": self.d_out[ctx.last_step & 1]}
+
     def e2e_setup(self, ctx):
         capi = ctx.capi
         self.Be = min(self.B, 4)
@@ -461,6 +471,9 @@ class C4:
         ctx.extra_events.setdefault("mips_box", []).append((m0, m1))
         return e0, e1, self.d_out[i & 1]
 
+    def outputs(self, ctx):
+        return {"mip_chain_rgba8": self.d_chain, "bc3_blocks": self.d_out[ctx.last_step & 1]}
+
     def e2e_setup(self, ctx):
         capi = ctx.capi
         self.Be = min(self.B, 128)
@@ -587,6 +600,9 @@ class C5:
         ctx.extra_events.setdefault("convert_r32f_to_r8", []).append((r0, r1))
         return e0, e1, self.d_bc[i & 1]
 
+    def outputs(self, ctx):
+        return {"bc4_blocks": self.d_bc[ctx.last_step & 1], "r32f": self.d_f32, "r8_roundtrip": self.d_back}
+
     def e2e_setup(self, ctx):
         capi = ctx.capi
         n = self.W * self.H
@@ -649,6 +665,28 @@ class C5:
 WORKLOADS = {"c2": C2, "c3": C3, "c4": C4, "c5": C5}
 
 
+DUMP_BUDGET = 60 << 20      # bytes of float32 over all dumped outputs
+
+
+def dump_outputs(outputs, path, torch):
+    """writes each output as float32 (bytes as their values 0..255): whole, or -- when the outputs together exceed DUMP_BUDGET --
+    the same seeded sample of 16-byte rows in every run; returns what was written"""
+    os.makedirs(path, exist_ok=True)
+    written = {}
+    for name, t in sorted(outputs.items()):
+        per_row = 16 // t.element_size()
+        flat = t.reshape(-1)
+        flat = flat[: flat.numel() // per_row * per_row].reshape(-1, per_row)
+        n, cap = flat.shape[0], DUMP_BUDGET // len(outputs) // (per_row * 4)
+        if n > cap:
+            idx = np.sort(np.random.default_rng(0).choice(n, cap, replace=False))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+        a = flat.float().cpu().numpy()
+        np.save(os.path.join(path, name + ".npy"), a)
+        written[name] = {"rows": int(a.shape[0]), "of_rows": int(n), "row_bytes": 16, "sample_seed": 0 if a.shape[0] < n else None}
+    return written
+
+
 # =====================================================================================================================
 def run_reference(args):
     """--impl reference: the reference's own CPU implementation of the path (oracle/_ref = the unmodified sources), all host threads,
@@ -688,6 +726,7 @@ def main():
     ap.add_argument("--config", default="c2", choices=sorted(WORKLOADS))
     ap.add_argument("--batch", type=int, default=0, help="images per GPU per step (c4: images in the whole batch); 0 = the config's default")
     ap.add_argument("--gather", default="nccl", choices=["nccl", "none"], help="end-of-step collection of the packed blocks at N>1")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)
@@ -771,6 +810,7 @@ def main():
     launches = capi.launch_count() - launches0
     tma_timed = capi.tma_launch_count() - tma0
     clocks = sampler.stop() if rank == 0 else None
+    dumped = dump_outputs(wl.outputs(ctx), args.dump_outputs, torch) if (args.dump_outputs and rank == 0) else None
     ms_total = e0.elapsed_time(e1)
     kern_ms = float(np.mean([a.elapsed_time(b) for a, b in kern_ev]))
     extra_ms = {k: float(np.mean([a.elapsed_time(b) for a, b in v])) for k, v in ctx.extra_events.items()}
@@ -807,13 +847,21 @@ def main():
     if rank == 0:
         pk, pk_kind = peaks()
         achieved = wl.algo_bytes() / (kern_ms * 1e-3) / 1e9
-        ref = load_ref()
-        u, sec, desc = wl.reference_step(ref)
-        threads = ref.threads()
-        ref.L.ref_omp_set_threads(1)
-        u1, sec1, _ = wl.reference_step(ref, **wl.small_sample)
-        ref.L.ref_omp_set_threads(threads)
-        parity = wl.parity(ctx, ref)
+        from tests import oracle_lib
+        cpu_baseline = parity = None
+        if os.path.exists(oracle_lib.REF_SO):
+            ref = load_ref()
+            u, sec, desc = wl.reference_step(ref)
+            threads = ref.threads()
+            ref.L.ref_omp_set_threads(1)
+            u1, sec1, _ = wl.reference_step(ref, **wl.small_sample)
+            ref.L.ref_omp_set_threads(threads)
+            parity = wl.parity(ctx, ref)
+            cpu_baseline = {"value": u / sec / 1e6, "unit": "Mtexels/s", "cores": threads, "kind": "reference",
+                            "sample": desc + ", %.2f s" % sec, "threads": threads, "proc_bind": os.environ.get("OMP_PROC_BIND"),
+                            "one_thread_value": u1 / sec1 / 1e6, "per_core_scaling": (u / sec) / (u1 / sec1) / max(threads, 1),
+                            "note": "the reference sources are compiled against a scalar DirectXMath stand-in (oracle/compat), not the SSE2 DirectXMath; "
+                                    "bounded sample, not the full workload"}
         traffic = None
         rd, wr = ncu_metric(wl.ncu_file, "dram__bytes_read.sum"), ncu_metric(wl.ncu_file, "dram__bytes_write.sum")
         if rd is not None and wr is not None:
@@ -840,13 +888,11 @@ def main():
                          "note": wl.bound_note},
             "kernels": dict({wl.kernel: kern_ms}, **extra_ms),
             "alternates": alternates,
-            "cpu_baseline": {"value": u / sec / 1e6, "unit": "Mtexels/s", "cores": threads, "kind": "reference",
-                             "sample": desc + ", %.2f s" % sec, "threads": threads, "proc_bind": os.environ.get("OMP_PROC_BIND"),
-                             "one_thread_value": u1 / sec1 / 1e6, "per_core_scaling": (u / sec) / (u1 / sec1) / max(threads, 1),
-                             "note": "the reference sources are compiled against a scalar DirectXMath stand-in (oracle/compat), not the SSE2 DirectXMath; "
-                                     "bounded sample, not the full workload"},
+            "cpu_baseline": cpu_baseline,
             "parity": parity,
         }
+        if dumped is not None:
+            out["dumped_outputs"] = {"dir": args.dump_outputs, "arrays": dumped}
         print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

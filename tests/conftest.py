@@ -31,10 +31,13 @@ def pytest_collection_modifyitems(config, items):
 
 @pytest.fixture(scope="session")
 def oracle():
-    """ctypes handle on oracle/_ref/libdxtex_ref.so (the unmodified reference, built by oracle/Makefile).
-    Built here when /root/reference is mounted; on the GPU box the prebuilt .so travels with the repo."""
+    """The reference's answers (tests/golden/reference_calls.npz).  With DXB_RECORD_REFERENCE=<file> the calls go to the
+    reference build instead (oracle/_ref/libdxtex_ref.so, oracle/Makefile) and are recorded into <file> at the end of the session."""
     from tests import oracle_lib
-    return oracle_lib.load_ref()
+    ref = oracle_lib.load_reference_answers()
+    yield ref
+    if isinstance(ref, oracle_lib.Recorder):
+        ref.save(os.environ["DXB_RECORD_REFERENCE"])
 
 
 @pytest.fixture(scope="session")

@@ -1,6 +1,9 @@
-"""TEST INFRASTRUCTURE: ctypes access to the oracle (oracle/_ref/libdxtex_ref.so = the unmodified reference
-sources) and to the host lock-step emulator of our own kernels (tests/emul).  Never imported by the product."""
+"""TEST INFRASTRUCTURE: the reference's answers to the calls the tests make (tests/golden/reference_calls.npz, replayed by
+`Recorded`), ctypes access to the oracle that recorded them (oracle/_ref/libdxtex_ref.so = the unmodified reference sources,
+`Ref`) and the host lock-step emulator of our own kernels (tests/emul).  Never imported by the product."""
 import ctypes as C
+import hashlib
+import json
 import os
 import subprocess
 
@@ -9,15 +12,14 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libdxtex_ref.so")
 EMUL_SO = os.path.join(ROOT, "tests", "emul", "_build", "libdxb_emul.so")
+CALLS = os.path.join(ROOT, "tests", "golden", "reference_calls.npz")
 
 from directxtex_b200 import formats as F
 
 
 def build_ref():
-    if os.path.isdir("/root/reference/DirectXTex"):
-        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle")], check=True)
     if not os.path.exists(REF_SO):
-        raise RuntimeError("oracle/_ref/libdxtex_ref.so missing and /root/reference not mounted: cannot build the oracle")
+        raise RuntimeError("oracle/_ref/libdxtex_ref.so missing: build it with `make -C oracle REF=<DirectXTex checkout>`")
     return REF_SO
 
 
@@ -153,6 +155,141 @@ class Ref:
         assert hr == 0
         return out[:F.BLOCK_BYTES[fmt]]
 
+    def mipchain_layout(self, fmt, w, h, levels=0):
+        """(hr, level count, total bytes, [(offset, width, height, row pitch) per level])"""
+        A = C.c_size_t * 16
+        nl, tot = C.c_size_t(), C.c_size_t()
+        off, ws, hs, ps = A(), A(), A(), A()
+        self.L.ref_mipchain_layout.argtypes = [C.c_uint32, C.c_size_t, C.c_size_t, C.c_size_t, C.POINTER(C.c_size_t), C.POINTER(C.c_size_t)] + [C.POINTER(C.c_size_t)] * 4 + [C.c_size_t]
+        hr = self.L.ref_mipchain_layout(fmt, w, h, levels, nl, tot, off, ws, hs, ps, 16)
+        return F.hr_u32(hr), nl.value, tot.value, [[off[i], ws[i], hs[i], ps[i]] for i in range(nl.value)]
+
+    def bc7_block_sse(self, src_f32, w, h, flags=0):
+        """(hr, per-block sum of squared 8-bit RGBA differences of the reference encoder's BC7 blocks, float32 (h/4, w/4))"""
+        hr, blocks = self.compress(src_f32, w, h, 2, 98, flags)
+        d = self.decode_blocks(98, blocks, w, h).astype(np.float64) * 255.0 - bc7_ldr(src_f32).astype(np.float64)
+        return hr, (d ** 2).reshape(h // 4, 4, w // 4, 4, 4).sum((1, 3, 4)).astype(np.float32)
+
+
+def _digest(a):
+    return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()[:16]
+
+
+class Digest:
+    """A reference output (bytes) kept as a SHA-256 prefix and its length instead of the bytes: `same` compares an array with it."""
+
+    def __init__(self, hexdigest, nbytes):
+        self.hex, self.nbytes, self.size = hexdigest, nbytes, nbytes
+
+    def __repr__(self):
+        return "Digest(%s)" % self.hex
+
+
+def same(a, b):
+    """np.array_equal for arrays; byte equality of the other side where one side is a Digest"""
+    if isinstance(a, Digest) or isinstance(b, Digest):
+        return (a.hex if isinstance(a, Digest) else _digest(a)) == (b.hex if isinstance(b, Digest) else _digest(b))
+    return np.array_equal(a, b)
+
+
+def same_concat(got, wants, sizes):
+    """`same` for an output made of consecutive pieces of the given byte sizes"""
+    offs = np.cumsum([0] + list(sizes))
+    return got.size == offs[-1] and all(same(got[o:o + n], w) for o, n, w in zip(offs, sizes, wants))
+
+
+def _call_key(name, args, kwargs):
+    h = hashlib.sha256(name.encode())
+    for a in list(args) + [kwargs[k] for k in sorted(kwargs)]:
+        if isinstance(a, np.ndarray):
+            a = np.ascontiguousarray(a)
+            h.update(("%s%s" % (a.dtype.str, a.shape)).encode())
+            h.update(a.tobytes())
+        elif isinstance(a, (float, np.floating)):
+            h.update(repr(float(a)).encode())
+        else:
+            h.update(repr(int(a)).encode())
+    h.update(repr(sorted(kwargs)).encode())
+    return h.hexdigest()[:16]
+
+
+def _encode(v, full, arrays):
+    if isinstance(v, np.ndarray):
+        d = _digest(v)
+        if full:
+            arrays["a_" + d] = v
+            return {"a": d}
+        return {"d": d, "n": int(v.nbytes)}
+    if isinstance(v, (list, tuple)):
+        return [_encode(x, full, arrays) for x in v]
+    return int(v)
+
+
+def _decode(v, z):
+    if isinstance(v, dict):
+        return z["a_" + v["a"]] if "a" in v else Digest(v["d"], v["n"])
+    if isinstance(v, list):
+        return [_decode(x, z) for x in v]
+    return v
+
+
+class Recorded:
+    """The reference's answers, replayed from tests/golden/reference_calls.npz: the same methods as `Ref`, looked up by a hash
+    of the method name and every argument.  Array outputs come back as `Digest`s, or as arrays where the caller passes
+    full=True (the tests that measure a difference instead of asserting equality)."""
+
+    def __init__(self, path=CALLS):
+        self.z = np.load(path)
+        self.calls = json.loads(bytes(self.z["calls"]).decode())
+
+    def __getattr__(self, name):
+        if name.startswith("_") or name in ("z", "calls"):
+            raise AttributeError(name)
+
+        def call(*args, full=False, **kwargs):
+            key = _call_key(name, args, kwargs)
+            if key not in self.calls:
+                raise KeyError("no recorded reference answer for %s with these arguments (tests/golden/reference_calls.npz is recorded "
+                               "by running the suite with DXB_RECORD_REFERENCE set, see tests/conftest.py)" % name)
+            return tuple(_decode(v, self.z) for v in self.calls[key])
+        return call
+
+
+class Recorder:
+    """Wraps the live `Ref` and records each call as `Recorded` will replay it; `save` writes the file.  Callers get what the
+    replay gives, so a recording run exercises the same comparisons as a replay."""
+
+    def __init__(self, ref):
+        self.ref, self.calls, self.arrays = ref, {}, {}
+
+    def __getattr__(self, name):
+        if name.startswith("_") or name in ("ref", "calls", "arrays"):
+            raise AttributeError(name)
+
+        def call(*args, full=False, **kwargs):
+            rec = [_encode(v, full, self.arrays) for v in getattr(self.ref, name)(*args, **kwargs)]
+            self.calls[_call_key(name, args, kwargs)] = rec
+            return tuple(_decode(v, self.arrays) for v in rec)
+        return call
+
+    def save(self, path):
+        old = Recorded(path) if os.path.exists(path) else None
+        calls = dict(old.calls) if old else {}
+        arrays = {k: old.z[k] for k in old.z.files if k.startswith("a_")} if old else {}
+        calls.update(self.calls)
+        arrays.update(self.arrays)
+        used = {"a_" + v["a"] for rec in calls.values() for v in _flat(rec) if isinstance(v, dict) and "a" in v}
+        np.savez_compressed(path, calls=np.frombuffer(json.dumps(calls, sort_keys=True).encode(), np.uint8),
+                            **{k: v for k, v in arrays.items() if k in used})
+
+
+def _flat(v):
+    if isinstance(v, list):
+        for x in v:
+            yield from _flat(x)
+    else:
+        yield v
+
 
 class Emul:
     def __init__(self, path):
@@ -183,6 +320,13 @@ class Emul:
         hr = self.L.emul_decompress(blocks.ctypes.data, w, h, bc_fmt, dst_fmt, out.ctypes.data)
         return F.hr_u32(hr), out
 
+    def decode_blocks(self, fmt, blocks, w, h):
+        """BC blocks -> float32 image (h, w, 4): Decompress to R32G32B32A32_FLOAT, which the tests hold bit-exact to the reference
+        decoder (test_emulator_decompress_bit_exact)"""
+        hr, out = self.decompress(blocks, w, h, fmt, F.DXGI_FORMAT_R32G32B32A32_FLOAT)
+        assert hr == 0
+        return out.view(np.float32).reshape(h, w, 4)
+
     def generate_mipmaps(self, src, w, h, fmt, filter=0, levels=0):
         layout, total = F.mip_chain_layout(fmt, w, h, levels)
         chain = np.zeros(total, np.uint8)
@@ -205,6 +349,12 @@ class Emul:
 
 def load_ref():
     return Ref(build_ref())
+
+
+def load_reference_answers():
+    """`Recorded`, or a `Recorder` on the reference build when DXB_RECORD_REFERENCE names the file to record into"""
+    path = os.environ.get("DXB_RECORD_REFERENCE")
+    return Recorder(load_ref()) if path else Recorded()
 
 
 def load_emul():

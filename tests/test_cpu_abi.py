@@ -1,17 +1,18 @@
 """CPU suite: the C++ mirror against the reference's OWN public header.
-(1) tests/cpp/abi_probe.cpp is compiled once against /root/reference/DirectXTex/DirectXTex.h (through oracle/compat) and once against
-    directxtex_b200/host/DirectXTexB200.h: sizeof / offsetof of Image, TexMetadata, ScratchImage, Blob, CompressOptions, ConvertOptions and
-    the values of every public enumerator the path uses must print identically.
+(1) tests/cpp/abi_probe.cpp is compiled against directxtex_b200/host/DirectXTexB200.h: sizeof / offsetof of Image, TexMetadata, ScratchImage,
+    Blob, CompressOptions, ConvertOptions and the values of every public enumerator the path uses must print what the same probe prints
+    compiled against the reference's DirectXTex.h (through oracle/compat).
 (2) the mangled symbols libdxtex_b200.so exports for the mirrored functions must be exported by the reference build
     (oracle/_ref/libdxtex_ref.so) under exactly the same name, i.e. the signatures match the reference's.
-Where /root/reference is not mounted (GPU box) the committed snapshot tests/golden/abi_reference.txt stands in for the reference side."""
+The reference side is the committed snapshots under tests/golden/.  With DXB_REFERENCE_SRC=<the reference's DirectXTex directory> (and
+oracle/_ref built from it) the probes are also built against the reference and the snapshots rewritten from them."""
 import os
 import subprocess
 
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference/DirectXTex"
+REF = os.environ.get("DXB_REFERENCE_SRC", "")
 SNAP = os.path.join(ROOT, "tests", "golden", "abi_reference.txt")
 SNAP_SYMS = os.path.join(ROOT, "tests", "golden", "abi_reference_symbols.txt")
 CXX = "/usr/bin/g++" if os.path.exists("/usr/bin/g++") else "g++"

@@ -8,6 +8,7 @@ import pytest
 
 from directxtex_b200 import capi, formats as F, synth
 from tests import golden_util, oracle_lib, tolerance
+from tests.oracle_lib import same, same_concat
 
 pytestmark = pytest.mark.gpu
 
@@ -22,14 +23,14 @@ def test_bc15_golden():
     for name, src, meta, exp in golden_util.cases("compress_"):
         w, h, sf, df, flags = (int(v) for v in meta)
         got = capi.compress(src, w, h, sf, df, flags)
-        assert np.array_equal(got, exp), name
+        assert same(got, exp), name
     assert capi.launch_count() > n0          # the CUDA kernels really ran
 
 
 def test_config1_bc1_matches_reference_hash():
     img = synth.c1_rgba8(256, 256)
     got = capi.compress(img, 256, 256, 28, 71)
-    assert np.array_equal(got, golden_util.load()["config1_bc1_out"])
+    assert same(got, golden_util.load()["config1_bc1_out"])
 
 
 @pytest.mark.parametrize("df", [71, 74, 77, 80, 81, 83, 84])
@@ -41,7 +42,7 @@ def test_bc15_vs_oracle_random(oracle, df):
         for flags in (0, F.TEX_COMPRESS_UNIFORM, F.TEX_COMPRESS_DITHER, F.TEX_COMPRESS_PARALLEL):
             hr, want = oracle.compress(src, w, h, sf, df, flags & ~F.TEX_COMPRESS_PARALLEL)
             got = capi.compress(src, w, h, sf, df, flags)
-            assert hr == 0 and np.array_equal(got, want), (w, h, sf, df, hex(flags))
+            assert hr == 0 and same(got, want), (w, h, sf, df, hex(flags))
 
 
 def test_bc1_threshold_and_structured(oracle):
@@ -49,7 +50,7 @@ def test_bc1_threshold_and_structured(oracle):
     for thr in (0.0, 0.25, 0.5, 0.75, 1.0):
         hr, want = oracle.compress(img, 128, 128, 28, 71, 0, threshold=thr)
         got = capi.compress(img, 128, 128, 28, 71, 0, threshold=thr)
-        assert hr == 0 and np.array_equal(got, want), thr
+        assert hr == 0 and same(got, want), thr
 
 
 def test_compress_array_batch(oracle):
@@ -58,7 +59,7 @@ def test_compress_array_batch(oracle):
     outs = capi.compress_array(srcs, 40, 24, 28, 77)
     for s, o in zip(srcs, outs):
         hr, want = oracle.compress(s, 40, 24, 28, 77)
-        assert hr == 0 and np.array_equal(o, want)
+        assert hr == 0 and same(o, want)
 
 
 def test_bc7_bc6h_array_batch_equals_single_images(emul):
@@ -72,20 +73,20 @@ def test_bc7_bc6h_array_batch_equals_single_images(emul):
         outs = capi.compress_array(srcs, w, h, 2, dfmt)
         for s_, o in zip(srcs, outs):
             he, want = emul.compress(s_, w, h, 2, dfmt)
-            assert he == 0 and np.array_equal(o, want), dfmt
+            assert he == 0 and same(o, want), dfmt
 
 
 def test_convert_golden_and_random(oracle):
     for name, src, meta, exp in golden_util.cases("convert_"):
         w, h, sf, df, fl = (int(v) for v in meta)
         got = capi.convert(src, w, h, sf, df, fl)
-        assert np.array_equal(got, exp), name
+        assert same(got, exp), name
     rng = np.random.default_rng(4)
     for (sf, df) in [(61, 41), (41, 61), (28, 2), (2, 28), (10, 28), (2, 10), (28, 87)]:
         src = oracle_lib.random_image(sf, 257, 63, rng)
         hr, want = oracle.convert(src, 257, 63, sf, df)
         got = capi.convert(src, 257, 63, sf, df)
-        assert hr == 0 and np.array_equal(got, want), (sf, df)
+        assert hr == 0 and same(got, want), (sf, df)
 
 
 def test_convert_ordered_dither(oracle):
@@ -99,11 +100,11 @@ def test_convert_ordered_dither(oracle):
             src = oracle_lib.random_image(sf, 37, 9, rng)
             hr, want = oracle.convert(src, 37, 9, sf, df, F.TEX_FILTER_DITHER)
             got = capi.convert(src, 37, 9, sf, df, F.TEX_FILTER_DITHER)
-            assert hr == 0 and np.array_equal(got, want), (sf, df)
+            assert hr == 0 and same(got, want), (sf, df)
     src = rng.random((1102, 2048, 4), dtype=np.float32)
     hr, want = oracle.convert(src, 2048, 1102, 2, 28, F.TEX_FILTER_DITHER)
     got = capi.convert(src, 2048, 1102, 2, 28, F.TEX_FILTER_DITHER)
-    assert hr == 0 and np.array_equal(got, want)
+    assert hr == 0 and same(got, want)
 
 
 def test_convert_error_diffusion_dither(oracle):
@@ -116,7 +117,7 @@ def test_convert_error_diffusion_dither(oracle):
                 src = oracle_lib.random_image(sf, w, h, rng)
                 hr, want = oracle.convert(src, w, h, sf, df, fl)
                 got = capi.convert(src, w, h, sf, df, fl)
-                assert hr == 0 and np.array_equal(got, want), (sf, df, w, h, hex(fl))
+                assert hr == 0 and same(got, want), (sf, df, w, h, hex(fl))
 
 
 def test_convert_exhaustive_small_domains(oracle):
@@ -128,13 +129,13 @@ def test_convert_exhaustive_small_domains(oracle):
         for df in (2, 41):
             hr, want = oracle.convert(src, w, h, sf, df)
             got = capi.convert(src, w, h, sf, df)
-            assert hr == 0 and np.array_equal(got, want), (sf, df)
+            assert hr == 0 and same(got, want), (sf, df)
 
 
 def test_convert_srgb_within_one_code(oracle):
     rng = np.random.default_rng(5)
     src = oracle_lib.random_image(29, 64, 16, rng)
-    hr, want = oracle.convert(src, 64, 16, 29, 28)
+    hr, want = oracle.convert(src, 64, 16, 29, 28, full=True)
     got = capi.convert(src, 64, 16, 29, 28)
     assert hr == 0 and np.abs(got.astype(int) - want.astype(int)).max() <= 1
 
@@ -145,7 +146,7 @@ def test_mips_golden():
         if h == 1 and (fl & 0xF00000) == F.TEX_FILTER_BOX:
             continue
         got, _ = capi.generate_mipmaps(src, w, h, fmt, fl)
-        assert np.array_equal(got, exp), name
+        assert same(got, exp), name
 
 
 @pytest.mark.parametrize("fl", [F.TEX_FILTER_BOX, F.TEX_FILTER_LINEAR, F.TEX_FILTER_CUBIC, F.TEX_FILTER_TRIANGLE, F.TEX_FILTER_POINT, 0,
@@ -159,7 +160,7 @@ def test_mips_vs_oracle(oracle, fl):
         src = oracle_lib.random_image(fmt, w, h, rng)
         hr, want = oracle.generate_mipmaps(src, w, h, fmt, fl)
         got, _ = capi.generate_mipmaps(src, w, h, fmt, fl)
-        assert hr == 0 and np.array_equal(got, want), (fmt, w, h, hex(fl))
+        assert hr == 0 and same(got, want), (fmt, w, h, hex(fl))
 
 
 @pytest.mark.parametrize("fl", [0, F.TEX_FILTER_POINT, F.TEX_FILTER_BOX, F.TEX_FILTER_LINEAR, F.TEX_FILTER_CUBIC, F.TEX_FILTER_TRIANGLE,
@@ -174,7 +175,7 @@ def test_resize_vs_oracle(oracle, fl):
         src = oracle_lib.random_image(fmt, w, h, rng)
         hr, want = oracle.resize(src, w, h, fmt, nw, nh, fl)
         got = capi.resize(src, w, h, fmt, nw, nh, fl)
-        assert hr == 0 and np.array_equal(got, want), (fmt, w, h, nw, nh, hex(fl))
+        assert hr == 0 and same(got, want), (fmt, w, h, nw, nh, hex(fl))
 
 
 @pytest.mark.parametrize("flags", [0, 0x1, 0x2, 0x3])
@@ -184,13 +185,13 @@ def test_premultiply_alpha_vs_oracle(oracle, flags):
     rng = np.random.default_rng(23)
     for (fmt, w, h) in [(28, 64, 32), (87, 37, 5), (2, 33, 9), (10, 40, 8), (11, 16, 16), (24, 24, 8), (29, 64, 16)]:
         src = oracle_lib.random_image(fmt, w, h, rng)
-        hr, want = oracle.premultiply_alpha(src, w, h, fmt, flags)
+        hr, want = oracle.premultiply_alpha(src, w, h, fmt, flags, full=(fmt == 29 and not (flags & 1)))
         got = capi.premultiply_alpha(src, w, h, fmt, flags)
         assert hr == 0
         if fmt == 29 and not (flags & 1):
             assert np.abs(got.astype(np.int32) - want.astype(np.int32)).max() <= 1, (fmt, flags)
         else:
-            assert np.array_equal(got, want), (fmt, w, h, flags)
+            assert same(got, want), (fmt, w, h, flags)
     with pytest.raises(capi.DxTexError) as e:
         capi.premultiply_alpha(np.zeros((8, 8), np.uint8), 8, 8, 61, 0)            # R8 has no alpha
     assert e.value.hr == F.HRESULT_E_NOT_SUPPORTED
@@ -208,18 +209,19 @@ def _alpha_test_image(fmt, w, h, rng):
     return img.astype(np.float16) if fmt == 10 else img
 
 
-def test_scale_mipmaps_alpha_for_coverage(oracle):
+def test_scale_mipmaps_alpha_for_coverage(oracle, emul):
     """SURVEY 8(f) rank 4: GenerateMipMaps -> ScaleMipMapsAlphaForCoverage (texconv -keepcoverage), bit-exact vs the reference."""
     rng = np.random.default_rng(47)
     for fmt, w, h in [(28, 128, 128), (28, 48, 20), (2, 32, 32), (87, 16, 64), (10, 33, 17), (29, 64, 64)]:
         img = _alpha_test_image(fmt, w, h, rng)
         for ref in (0.5, 0.25):
             hr, plain, want = oracle.mips_alpha_coverage(img, w, h, fmt, ref)
-            got = capi.scale_mipmaps_alpha_for_coverage(plain, w, h, fmt, ref)
-            assert hr == 0 and np.array_equal(got, want), (fmt, w, h, ref)
+            hp, chain = emul.generate_mipmaps(img, w, h, fmt)       # the reference's plain chain, bit for bit
+            got = capi.scale_mipmaps_alpha_for_coverage(chain, w, h, fmt, ref)
+            assert hr == 0 and hp == 0 and same(chain, plain) and same(got, want), (fmt, w, h, ref)
 
 
-def test_bc7_equals_emulator_and_quality(oracle, emul):
+def test_bc7_equals_emulator_and_quality(emul):
     """GPU BC7 == host lock-step emulator (same source, explicit fmaf, -fmad=false) bit for bit, and
     MSE <= 1.02 x the reference CPU encoder's MSE (golden anchor) on each test image."""
     z = golden_util.load()
@@ -231,14 +233,14 @@ def test_bc7_equals_emulator_and_quality(oracle, emul):
         he, em = emul.compress(img, w, h, 2, 98)
         assert he == 0
         nd = int((got.reshape(-1, 16) != em.reshape(-1, 16)).any(1).sum())
-        mse = oracle_lib.mse255(oracle.decode_blocks(98, got, w, h), img)
+        mse = oracle_lib.mse255(emul.decode_blocks(98, got, w, h), img)
         ref_mse = float(z["bc7_%d_refmse" % j][0])
         assert mse <= ref_mse * 1.02, (kind, mse, ref_mse)
         assert nd == 0, "%d of %d blocks differ from the emulator" % (nd, got.size // 16)
 
 
 @pytest.mark.parametrize("kind,flags", tolerance.bc7_cases())
-def test_bc7_contract_per_class_on_device(oracle, emul, kind, flags):
+def test_bc7_contract_per_class_on_device(emul, kind, flags):
     """Every content class of the tolerance corpus at 256^2: the CUDA encoder's blocks are bit-identical to the host emulator's
     and meet the BC7 contract (tests/tolerance.py) against the reference encoder's per-block errors (committed golden)."""
     n = tolerance.SIZE
@@ -248,11 +250,11 @@ def test_bc7_contract_per_class_on_device(oracle, emul, kind, flags):
     assert he == 0
     nd = int((got.reshape(-1, 16) != em.reshape(-1, 16)).any(1).sum())
     assert nd == 0, "%s: %d of %d blocks differ from the emulator" % (kind, nd, got.size // 16)
-    tolerance.check_bc7(oracle, kind, flags, got)
+    tolerance.check_bc7(emul, kind, flags, got)
 
 
 @pytest.mark.parametrize("kind,fmt", tolerance.bc6h_cases())
-def test_bc6h_contract_per_class_on_device(oracle, emul, kind, fmt):
+def test_bc6h_contract_per_class_on_device(emul, kind, fmt):
     """As above for BC6H_UF16 / BC6H_SF16, including the float-domain bounds (sign-crossing content)."""
     n = tolerance.SIZE
     img = synth.content_hdr(kind, n, n, tolerance.SEED)
@@ -261,7 +263,7 @@ def test_bc6h_contract_per_class_on_device(oracle, emul, kind, fmt):
     assert he == 0
     nd = int((got.reshape(-1, 16) != em.reshape(-1, 16)).any(1).sum())
     assert nd == 0, "%s: %d blocks differ from the emulator" % (kind, nd)
-    tolerance.check_bc6h(oracle, kind, fmt, got)
+    tolerance.check_bc6h(emul, kind, fmt, got)
 
 
 @pytest.mark.parametrize("kind", ["cutout", "alpha_photo", "gradient", "c2"])
@@ -277,7 +279,7 @@ def test_bc7_device_equals_emulator_512(emul, kind):
     assert nd == 0, "%s: %d of %d blocks differ from the emulator" % (kind, nd, got.size // 16)
 
 
-def test_full_size_c2_bc7_mse_vs_reference_on_crop(oracle):
+def test_full_size_c2_bc7_mse_vs_reference_on_crop(oracle, emul):
     """BASELINE configs[1] "bit-check vs ref BC7 MSE": the 4096^2 image is compressed on the GPU; on a 512^2 aligned crop (16384
     blocks: the blocks of a crop are the blocks of the full image, test_full_size_c2_bc7_properties) the reference encoder runs
     here on the host and both streams are decoded by the reference decoder: MSE_gpu <= 1.02 x MSE_ref, < 1 % of blocks worse
@@ -287,22 +289,22 @@ def test_full_size_c2_bc7_mse_vs_reference_on_crop(oracle):
     y0, x0, s = 1536, 512, 512
     crop = np.ascontiguousarray(img[y0:y0 + s, x0:x0 + s])
     gpu_blocks = np.ascontiguousarray(a[y0 // 4:(y0 + s) // 4, x0 // 4:(x0 + s) // 4]).reshape(-1)
-    hr, ref_blocks = oracle.compress(crop, s, s, 2, 98, 0)
+    hr, theirs = oracle.bc7_block_sse(crop, s, s, 0, full=True)
     assert hr == 0
-    ours, theirs = tolerance.bc7_block_sse(oracle, gpu_blocks, crop), tolerance.bc7_block_sse(oracle, ref_blocks, crop)
+    ours, theirs = tolerance.bc7_block_sse(emul, gpu_blocks, crop), theirs.astype(np.float64)
     assert ours.sum() <= 1.02 * theirs.sum(), ours.sum() / theirs.sum()
     assert float((ours > 2.0 * theirs + 16.0).mean()) < 0.01
 
 
-def test_bc7_rgba8_source_partial_blocks_and_quick(oracle, emul):
+def test_bc7_rgba8_source_partial_blocks_and_quick(emul):
     rng = np.random.default_rng(8)
     for (w, h) in [(5, 7), (1, 1), (30, 18)]:
         src = oracle_lib.random_image(28, w, h, rng)
         for flags in (0, F.TEX_COMPRESS_BC7_QUICK):
             got = capi.compress(src, w, h, 28, 98, flags)
             he, em = emul.compress(src, w, h, 28, 98, flags)
-            assert he == 0 and np.array_equal(got, em), (w, h, flags)
-            dec = oracle.decode_blocks(98, got, w, h)      # decodable by the reference decoder
+            assert he == 0 and same(got, em), (w, h, flags)
+            dec = emul.decode_blocks(98, got, w, h)      # decodable (the decoder is bit-exact to the reference's)
             assert np.isfinite(dec).all()
 
 
@@ -329,7 +331,7 @@ def _tma_cases(emul, torch, rng):
             img[:, :48, 3] = 1.0
         got = capi.compress(img, w, h, 2, 98, flags)
         he, em = emul.compress(img, w, h, 2, 98, flags)
-        assert he == 0 and np.array_equal(got, em), (w, h, flags)
+        assert he == 0 and same(got, em), (w, h, flags)
     w, h, n = 72, 20, 3
     imgs = rng.random((n, h, w, 4), dtype=np.float32)
     st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -347,7 +349,7 @@ def _tma_cases(emul, torch, rng):
         out = d_out.cpu().numpy().reshape(n, sl)
         for i in range(n):
             he, em = emul.compress(imgs[i], w, h, 2, 98, 0)
-            assert he == 0 and np.array_equal(out[i], em), (pad, i)
+            assert he == 0 and same(out[i], em), (pad, i)
 
 
 def test_device_api_with_torch_pointers(oracle):
@@ -362,28 +364,28 @@ def test_device_api_with_torch_pointers(oracle):
     assert capi.lib.dxb200_compress_device(s, 1, 77, 0, 0.5, 1.0, d, C.c_void_p(st.cuda_stream)) == 0
     torch.cuda.synchronize()
     hr, want = oracle.compress(img, 128, 64, 28, 77)
-    assert hr == 0 and np.array_equal(d_out.cpu().numpy(), want)
+    assert hr == 0 and same(d_out.cpu().numpy(), want)
 
 
-def test_full_size_c2_bc7_properties(oracle, emul):
+def test_full_size_c2_bc7_properties(emul):
     """BASELINE configs[1] at full size (4096^2 RGBA32F -> BC7): size-independent properties.
     determinism; locality (the blocks of an aligned crop are identical to the same blocks of the full image);
     the crop equals the emulator; whole-image MSE sane (PSNR > 30 dB)."""
     img = synth.c2_rgba32f(4096, 4096)
     a = capi.compress(img, 4096, 4096, 2, 98)
     b = capi.compress(img, 4096, 4096, 2, 98)
-    assert np.array_equal(a, b)
+    assert same(a, b)
     y0, x0, s = 1024, 2048, 128
     crop = np.ascontiguousarray(img[y0:y0 + s, x0:x0 + s])
     cb = capi.compress(crop, s, s, 2, 98).reshape(s // 4, s // 4, 16)
     full = a.reshape(1024, 1024, 16)[y0 // 4:(y0 + s) // 4, x0 // 4:(x0 + s) // 4]
-    assert np.array_equal(cb, full)
+    assert same(cb, full)
     he, em = emul.compress(crop, s, s, 2, 98)
-    assert he == 0 and np.array_equal(cb.reshape(-1), em)
+    assert he == 0 and same(cb.reshape(-1), em)
     step = 8
     sub = a.reshape(1024, 1024, 16)[::step, ::step].reshape(-1, 16).copy()
-    dec = np.zeros((sub.shape[0], 16, 4), np.float32)
-    assert oracle.L.ref_decode_blocks(98, sub.ctypes.data, sub.shape[0], dec.ctypes.data) == 0
+    n = sub.shape[0]
+    dec = emul.decode_blocks(98, sub, 4 * n, 4).reshape(4, n, 4, 4).transpose(1, 0, 2, 3).reshape(n, 16, 4)
     src_blocks = img.reshape(1024, 4, 1024, 4, 4).transpose(0, 2, 1, 3, 4)[::step, ::step].reshape(-1, 16, 4)
     mse = float(((dec.astype(np.float64) * 255.0 - oracle_lib.bc7_ldr(src_blocks)) ** 2).mean())
     assert oracle_lib.psnr(mse) > 30.0, mse
@@ -396,14 +398,14 @@ def test_full_size_c5_bc4_and_convert_roundtrip(oracle):
     for by in (0, 777, 2047):
         rows = np.ascontiguousarray(img[by * 4:by * 4 + 4])
         hr, want = oracle.compress(rows, 8192, 4, 61, 80)
-        assert hr == 0 and np.array_equal(got[by].reshape(-1), want), by
+        assert hr == 0 and same(got[by].reshape(-1), want), by
     f = capi.convert(img, 8192, 8192, 61, 41)
-    assert np.array_equal(f.view(np.float32), (img.reshape(-1).astype(np.float32) / np.float32(255.0)))
+    assert same(f.view(np.float32), (img.reshape(-1).astype(np.float32) / np.float32(255.0)))
     back = capi.convert(f, 8192, 8192, 41, 61)
-    assert np.array_equal(back, img.reshape(-1))
+    assert same(back, img.reshape(-1))
 
 
-def test_bc6h_equals_emulator_and_quality(oracle, emul):
+def test_bc6h_equals_emulator_and_quality(emul):
     """GPU BC6H == host lock-step emulator bit for bit; error (reference metric) <= 1.02 x the reference CPU encoder's."""
     z = golden_util.load()
     for j in range(4):
@@ -413,7 +415,7 @@ def test_bc6h_equals_emulator_and_quality(oracle, emul):
         got = capi.compress(img, w, h, 2, fmt)
         he, em = emul.compress(img, w, h, 2, fmt)
         assert he == 0
-        err = oracle_lib.bc6h_int_mse(oracle.decode_blocks(fmt, got, w, h), img, fmt == 96)
+        err = oracle_lib.bc6h_int_mse(emul.decode_blocks(fmt, got, w, h), img, fmt == 96)
         assert err <= float(z["bc6h_%d_referr" % j][0]) * 1.02, (kind, err)
         nd = int((got.reshape(-1, 16) != em.reshape(-1, 16)).any(1).sum())
         assert nd == 0, "%d blocks differ from the emulator" % nd
@@ -426,12 +428,12 @@ def test_config3_rgba16f_cubic_chain_bc6h(oracle, emul):
     img = synth.c3_rgba16f(w, h)
     chain, layout = capi.generate_mipmaps(img, w, h, 10, F.TEX_FILTER_CUBIC)
     hr, want = oracle.generate_mipmaps(img, w, h, 10, F.TEX_FILTER_CUBIC)
-    assert hr == 0 and np.array_equal(chain, want)
+    assert hr == 0 and same(chain, want)
     for (off, lw, lh, row, sl) in layout[:4]:
         level = chain[off:off + sl]
         got = capi.compress(level, lw, lh, 10, 95)
         he, em = emul.compress(level, lw, lh, 10, 95)
-        assert he == 0 and np.array_equal(got, em)
+        assert he == 0 and same(got, em)
 
 
 DECOMPRESS_CASES = ((71, (28, 2)), (74, (28,)), (77, (28, 2)), (80, (61, 41)), (81, (63, 41)), (83, (49, 16)), (84, (51,)),
@@ -443,7 +445,7 @@ def _bc_inputs(oracle, bc, w, h, rng):
     nb = ((w + 3) // 4) * ((h + 3) // 4)
     yield rng.integers(0, 256, nb * F.BLOCK_BYTES[bc], dtype=np.uint8)
     src = rng.random((h, w, 4)).astype(np.float32) * (4.0 if bc in (95, 96) else 1.0) - (1.0 if bc in (81, 84, 96) else 0.0)
-    hr, blocks = oracle.compress(src, w, h, 2, bc, 0)
+    hr, blocks = oracle.compress(src, w, h, 2, bc, 0, full=True)
     assert hr == 0
     yield blocks
 
@@ -456,7 +458,7 @@ def test_decompress_bit_exact(oracle):
                 for df in dsts:
                     hr, want = oracle.decompress(blocks, w, h, bc, df)
                     got = capi.decompress(blocks, w, h, bc, df)
-                    assert hr == 0 and np.array_equal(got, want), (bc, df, w, h)
+                    assert hr == 0 and same(got, want), (bc, df, w, h)
 
 
 def test_compress_decompress_round_trip_full_size():
@@ -478,9 +480,9 @@ def test_mipmaps_compress_equals_two_calls_and_reference(oracle):
         for src, got in zip(srcs, outs):
             chain, layout = capi.generate_mipmaps(src, w, h, 28, 0)
             hr, rchain = oracle.generate_mipmaps(src, w, h, 28, 0)
-            assert hr == 0 and np.array_equal(chain, rchain)
-            want = np.concatenate([oracle.compress(rchain[off:off + sl], lw, lh, 28, 77)[1] for (off, lw, lh, row, sl) in layout])
-            assert np.array_equal(got, want), (w, h)
+            assert hr == 0 and same(chain, rchain)
+            want = [oracle.compress(chain[off:off + sl], lw, lh, 28, 77)[1] for (off, lw, lh, row, sl) in layout]
+            assert same_concat(got, want, [F.compute_pitch(77, lw, lh)[1] for (off, lw, lh, row, sl) in layout]), (w, h)
 
 
 def test_concurrent_host_calls_from_threads(oracle):
@@ -499,27 +501,30 @@ def test_concurrent_host_calls_from_threads(oracle):
         t.join()
     for i, s_ in enumerate(srcs):
         hr, want = oracle.compress(s_, 512, 256, 28, 77 if i % 2 else 71)
-        assert hr == 0 and np.array_equal(res[i], want), i
+        assert hr == 0 and same(res[i], want), i
 
 
-def test_multi_device_sharding_inside_the_library(oracle):
+def test_multi_device_sharding_inside_the_library(oracle, emul):
     """dxb200_init_devices: array calls and mip chains are sharded over the GPUs inside one process; results unchanged"""
+    rng = np.random.default_rng(47)
+    srcs = [oracle_lib.random_image(28, 128, 64, rng) for _ in range(17)]       # 2 n + 1 images for up to 8 GPUs
+    layout, _ = F.mip_chain_layout(28, 128, 64, 0)
+    want_bc3 = [oracle.compress(s_, 128, 64, 28, 77) for s_ in srcs]
+    want_chain = [oracle.generate_mipmaps(s_, 128, 64, 28, 0) for s_ in srcs]
+    chains = [emul.generate_mipmaps(s_, 128, 64, 28, 0)[1] for s_ in srcs]        # equal to the reference's chains (asserted below)
+    want_bc1 = [[oracle.compress(c[off:off + sl], lw, lh, 28, 71)[1] for (off, lw, lh, row, sl) in layout] for c in chains]
     n = capi.lib.dxb200_device_count()
     if n < 2:
         pytest.skip("needs >= 2 GPUs")
+    srcs = srcs[:2 * n + 1]
     capi.init_devices(list(range(n)))
-    rng = np.random.default_rng(47)
-    srcs = [oracle_lib.random_image(28, 128, 64, rng) for _ in range(2 * n + 1)]
     outs = capi.compress_array(srcs, 128, 64, 28, 77)
-    for s_, o in zip(srcs, outs):
-        hr, want = oracle.compress(s_, 128, 64, 28, 77)
-        assert hr == 0 and np.array_equal(o, want)
+    for (hr, want), o in zip(want_bc3, outs):
+        assert hr == 0 and same(o, want)
     outs = capi.mipmaps_compress(srcs, 128, 64, 28, 71)
-    for s_, o in zip(srcs, outs):
-        hr, rchain = oracle.generate_mipmaps(s_, 128, 64, 28, 0)
-        layout, _ = F.mip_chain_layout(28, 128, 64, 0)
-        want = np.concatenate([oracle.compress(rchain[off:off + sl], lw, lh, 28, 71)[1] for (off, lw, lh, row, sl) in layout])
-        assert hr == 0 and np.array_equal(o, want)
+    for (hr, rchain), c, want, o in zip(want_chain, chains, want_bc1, outs):
+        assert hr == 0 and same(c, rchain)
+        assert same_concat(o, want, [F.compute_pitch(71, lw, lh)[1] for (off, lw, lh, row, sl) in layout])
 
 
 def test_next_tier_formats_vs_oracle(oracle):
@@ -532,21 +537,21 @@ def test_next_tier_formats_vs_oracle(oracle):
         for fl in (0, F.TEX_FILTER_FLOAT_X2BIAS):
             hr, want = oracle.convert(src, 133, 21, sf, df, fl)
             got = capi.convert(src, 133, 21, sf, df, fl)
-            assert hr == 0 and np.array_equal(got, want), (sf, df, hex(fl))
+            assert hr == 0 and same(got, want), (sf, df, hex(fl))
     src = oracle_lib.random_image(2, 64, 8, rng)
     for thr in (0.0, 0.25, 0.9):
         hr, want = oracle.convert(src, 64, 8, 2, 86, 0, threshold=thr)
         got = capi.convert(src, 64, 8, 2, 86, 0, threshold=thr)
-        assert hr == 0 and np.array_equal(got, want), thr
+        assert hr == 0 and same(got, want), thr
     for fmt in NEXT_TIER:
         src = oracle_lib.random_image(fmt, 40, 24, rng)
         for fl in (F.TEX_FILTER_POINT, F.TEX_FILTER_LINEAR, F.TEX_FILTER_CUBIC, F.TEX_FILTER_TRIANGLE, 0):
             hr, want = oracle.generate_mipmaps(src, 40, 24, fmt, fl)
             got, _ = capi.generate_mipmaps(src, 40, 24, fmt, fl)
-            assert hr == 0 and np.array_equal(got, want), (fmt, hex(fl))
+            assert hr == 0 and same(got, want), (fmt, hex(fl))
         for bc in (71, 77, 80, 83):
             hr, want = oracle.compress(src, 40, 24, fmt, bc)
-            assert hr == 0 and np.array_equal(capi.compress(src, 40, 24, fmt, bc), want), (fmt, bc)
+            assert hr == 0 and same(capi.compress(src, 40, 24, fmt, bc), want), (fmt, bc)
     with pytest.raises(capi.DxTexError) as e:
         capi.convert(oracle_lib.random_image(28, 16, 16, rng), 16, 16, 28, 85, F.TEX_FILTER_DITHER)
     assert e.value.hr == F.HRESULT_E_NOT_SUPPORTED

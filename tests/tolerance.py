@@ -52,17 +52,17 @@ def _blocks(a, n):
     return a.reshape(n // 4, 4, n // 4, 4, -1).sum((1, 3, 4))
 
 
-def bc7_block_sse(ref, blocks, img):
+def bc7_block_sse(decoder, blocks, img):
     n = img.shape[0]
-    dec = ref.decode_blocks(98, blocks, n, n).astype(np.float64) * 255.0
+    dec = decoder.decode_blocks(98, blocks, n, n).astype(np.float64) * 255.0
     src = oracle_lib.bc7_ldr(img).astype(np.float64)
     return _blocks((dec - src) ** 2, n)
 
 
-def bc6h_block_errors(ref, blocks, img, fmt):
+def bc6h_block_errors(decoder, blocks, img, fmt):
     n = img.shape[0]
     signed = fmt == 96
-    dec = ref.decode_blocks(fmt, blocks, n, n)
+    dec = decoder.decode_blocks(fmt, blocks, n, n)
     clip = np.clip(img[..., :3], -65504 if signed else 0, 65504)
     a = oracle_lib.bc6h_to_int(dec[..., :3], signed).astype(np.float64)
     s = oracle_lib.bc6h_to_int(clip, signed).astype(np.float64)
@@ -81,12 +81,12 @@ def check_input(key, img):
     assert bytes(golden()[key + "_sha1"]) == hashlib.sha1(img.tobytes()).digest(), "regenerated input differs from the golden's: " + key
 
 
-def check_bc7(ref, kind, flags, blocks):
-    """asserts the BC7 contract for `blocks` (our encoder's output for class `kind`); returns (ratio, bad fraction)"""
+def check_bc7(decoder, kind, flags, blocks):
+    """asserts the BC7 contract for `blocks` (our encoder's output for class `kind`, decoded by `decoder`); returns (ratio, bad fraction)"""
     key = bc7_key(kind, flags)
     img = synth.content_ldr(kind, SIZE, SIZE, SEED)
     check_input(key, img)
-    ours = bc7_block_sse(ref, blocks, img)
+    ours = bc7_block_sse(decoder, blocks, img)
     theirs = golden()[key + "_sse"].astype(np.float64)
     ratio = ours.sum() / max(theirs.sum(), 1e-9)
     bad = float((ours > 2.0 * theirs + 16.0).mean())
@@ -95,12 +95,12 @@ def check_bc7(ref, kind, flags, blocks):
     return ratio, bad
 
 
-def check_bc6h(ref, kind, fmt, blocks):
+def check_bc6h(decoder, kind, fmt, blocks):
     key = bc6h_key(kind, fmt)
     img = synth.content_hdr(kind, SIZE, SIZE, SEED)
     check_input(key, img)
     z = golden()
-    isse, fsse, fmax = bc6h_block_errors(ref, blocks, img, fmt)
+    isse, fsse, fmax = bc6h_block_errors(decoder, blocks, img, fmt)
     risse, rfsse, rfmax = z[key + "_isse"], z[key + "_fsse"], float(z[key + "_fmax"][0])
     npx = SIZE * SIZE * 3
     ratio = isse.sum() / max(risse.sum(), 1e-9)
