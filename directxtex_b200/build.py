@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_lib")
 OUT = os.path.join(OUT_DIR, "libdxtex_b200.so")
-SOURCES = [os.path.join(CSRC, f) for f in ("dxb_api.cu", "dxb_k_bc7.cu", "dxb_k_bc6h.cu", "dxb_k_bc15.cu", "dxb_k_decode.cu", "dxb_k_rows.cu")]
+SOURCES = [os.path.join(CSRC, f) for f in ("dxb_api.cu", "dxb_k_bc7.cu", "dxb_k_bc6h.cu", "dxb_k_bc15.cu", "dxb_k_decode.cu", "dxb_k_rows.cu", "dxb_k_analyze.cu")]
 HOST_SOURCES = [os.path.join(HERE, "host", "DirectXTexB200.cpp"), os.path.join(HERE, "host", "dxb_dds.cpp")]
 
 

@@ -16,6 +16,7 @@ SYMBOLS = [
     "dxb200_resize", "dxb200_resize_device", "dxb200_premultiply_alpha", "dxb200_premultiply_alpha_device",
     "dxb200_scale_mipmaps_alpha_for_coverage", "dxb200_scale_mipmaps_alpha_for_coverage_device",
     "dxb200_dds_encode_header", "dxb200_dds_save_memory", "dxb200_dds_get_metadata", "dxb200_dds_load_memory",
+    "dxb200_compute_mse", "dxb200_compute_mse_device", "dxb200_is_alpha_all_opaque", "dxb200_is_alpha_all_opaque_device",
 ]
 
 
@@ -87,7 +88,13 @@ def _load():
     lib.dxb200_dds_save_memory.argtypes = [IP, C.c_size_t, MP, C.c_uint32, C.c_void_p, C.c_size_t, SP]
     lib.dxb200_dds_get_metadata.argtypes = [C.c_void_p, C.c_size_t, C.c_uint32, MP, SP]
     lib.dxb200_dds_load_memory.argtypes = [C.c_void_p, C.c_size_t, C.c_uint32, IP, C.c_size_t]
-    for name in ("dxb200_dds_encode_header", "dxb200_dds_save_memory", "dxb200_dds_get_metadata", "dxb200_dds_load_memory"):
+    FP = C.POINTER(C.c_float)
+    lib.dxb200_compute_mse.argtypes = [IP, IP, C.c_size_t, C.c_uint32, FP, FP]
+    lib.dxb200_compute_mse_device.argtypes = [IP, IP, C.c_size_t, C.c_uint32, C.c_void_p, C.c_void_p]
+    lib.dxb200_is_alpha_all_opaque.argtypes = [IP, C.c_size_t, C.POINTER(C.c_int32)]
+    lib.dxb200_is_alpha_all_opaque_device.argtypes = [IP, C.c_size_t, C.c_void_p, C.c_void_p]
+    for name in ("dxb200_compute_mse", "dxb200_compute_mse_device", "dxb200_is_alpha_all_opaque", "dxb200_is_alpha_all_opaque_device",
+                 "dxb200_dds_encode_header", "dxb200_dds_save_memory", "dxb200_dds_get_metadata", "dxb200_dds_load_memory"):
         getattr(lib, name).restype = C.c_int32
     for name in ("dxb200_init", "dxb200_init_devices", "dxb200_initialized_devices", "dxb200_compress_ex", "dxb200_convert_ex", "dxb200_mipmaps_compress", "dxb200_device_count", "dxb200_compute_pitch", "dxb200_calculate_mip_levels", "dxb200_compress",
                  "dxb200_compress_device", "dxb200_decompress", "dxb200_decompress_device", "dxb200_convert",
@@ -320,3 +327,54 @@ def decompress(blocks, w, h, bc_fmt, dst_fmt):
     if hr != 0:
         raise DxTexError(hr, "dxb200_decompress")
     return out[:sl]
+
+
+# ------------------------------------------------------------------------------------------------
+# ComputeMSE / IsAlphaAllOpaque
+CMSE_DEFAULT, CMSE_IMAGE1_SRGB, CMSE_IMAGE2_SRGB = 0, 0x1, 0x2
+CMSE_IGNORE_RED, CMSE_IGNORE_GREEN, CMSE_IGNORE_BLUE, CMSE_IGNORE_ALPHA = 0x10, 0x20, 0x40, 0x80
+CMSE_IMAGE1_X2_BIAS, CMSE_IMAGE2_X2_BIAS = 0x100, 0x200
+
+
+def compute_mse_images(a, b, flags=0):
+    """dxb200_compute_mse of prepared Image structs (lists of equal length): returns (hr, mse float32[n], mseV float32[n, 4])."""
+    n = len(a)
+    mse, mse_v = np.zeros(n, np.float32), np.zeros((n, 4), np.float32)
+    hr = lib.dxb200_compute_mse(images(a), images(b), n, flags, mse.ctypes.data_as(C.POINTER(C.c_float)), mse_v.ctypes.data_as(C.POINTER(C.c_float)))
+    return F.hr_u32(hr), mse, mse_v
+
+
+def compute_mse(a, fmt_a, b, fmt_b, w, h, flags=0, pitch_a=0, pitch_b=0):
+    """DirectX::ComputeMSE of two host images (numpy buffers holding the rows); returns (mse, mseV[4]) as float32."""
+    a, b = np.ascontiguousarray(a), np.ascontiguousarray(b)
+    hr, mse, mse_v = compute_mse_images([make_image(_np_ptr(a), w, h, fmt_a, pitch_a)], [make_image(_np_ptr(b), w, h, fmt_b, pitch_b)], flags)
+    if hr != 0:
+        raise DxTexError(hr, "dxb200_compute_mse")
+    return mse[0], mse_v[0]
+
+
+def compute_mse_device(a, b, flags, out_ptr, stream=None):
+    """dxb200_compute_mse_device: a / b = Image structs holding device pointers, out_ptr = device float[5 n]; returns the HRESULT."""
+    return F.hr_u32(lib.dxb200_compute_mse_device(images(a), images(b), len(a), flags, out_ptr, stream))
+
+
+def is_alpha_all_opaque_images(imgs):
+    """dxb200_is_alpha_all_opaque of prepared Image structs (one format): returns (hr, opaque bool)."""
+    v = C.c_int32(-1)
+    hr = lib.dxb200_is_alpha_all_opaque(images(imgs), len(imgs), C.byref(v))
+    return F.hr_u32(hr), v.value == 1
+
+
+def is_alpha_all_opaque(pixels, layout, fmt):
+    """The IsAlphaAllOpaque scan of the images of one texture held in `pixels` at the (offset, w, h, rowPitch, slicePitch) entries
+    of `layout` (texture_layout / formats.mip_chain_layout); returns True / False."""
+    pixels = np.ascontiguousarray(pixels).view(np.uint8).reshape(-1)
+    hr, v = is_alpha_all_opaque_images([Image(lw, lh, fmt, row, sl, _np_ptr(pixels) + off) for (off, lw, lh, row, sl) in layout])
+    if hr != 0:
+        raise DxTexError(hr, "dxb200_is_alpha_all_opaque")
+    return v
+
+
+def is_alpha_all_opaque_device(imgs, out_ptr, stream=None):
+    """dxb200_is_alpha_all_opaque_device: imgs = Image structs holding device pointers, out_ptr = device int32; returns the HRESULT."""
+    return F.hr_u32(lib.dxb200_is_alpha_all_opaque_device(images(imgs), len(imgs), out_ptr, stream))

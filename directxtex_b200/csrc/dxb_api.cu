@@ -440,8 +440,11 @@ void split_bands(const dxb200_image* src, const dxb200_image* dst, size_t n, siz
     }
 }
 
+// dst == nullptr: the kernels write no image (IsAlphaAllOpaque); dstIn: dst[] is a second INPUT, copied up like src and not back
+// (ComputeMSE)
 template <typename LaunchFn>
-int32_t run_staged(const dxb200_image* src, const dxb200_image* dst, size_t n, LaunchFn fn, Progress* prog = nullptr, const size_t* units = nullptr)
+int32_t run_staged(const dxb200_image* src, const dxb200_image* dst, size_t n, LaunchFn fn, Progress* prog = nullptr, const size_t* units = nullptr,
+                   bool dstIn = false)
 {
     const size_t CHUNK = size_t(48) << 20;
     size_t i = 0; int slot = 0;
@@ -451,7 +454,7 @@ int32_t run_staged(const dxb200_image* src, const dxb200_image* dst, size_t n, L
         size_t inBytes = 0, outBytes = 0, k = i;
         while (k < n)
         {
-            const size_t a = (src[k].slicePitch + 255) & ~size_t(255), b = (dst[k].slicePitch + 255) & ~size_t(255);
+            const size_t a = (src[k].slicePitch + 255) & ~size_t(255), b = dst ? (dst[k].slicePitch + 255) & ~size_t(255) : 0;
             if (k > i && (inBytes + a + outBytes + b) > CHUNK) break;
             inBytes += a; outBytes += b; ++k;
         }
@@ -465,19 +468,22 @@ int32_t run_staged(const dxb200_image* src, const dxb200_image* dst, size_t n, L
         }
         hr = ensure_buffer(&t_v.lane->dIn[slot], &t_v.lane->dInCap[slot], inBytes); if (hr) break;
         hr = ensure_buffer(&t_v.lane->dOut[slot], &t_v.lane->dOutCap[slot], outBytes); if (hr) break;
-        std::vector<dxb200_image> ds(src + i, src + k), dd(dst + i, dst + k);
+        std::vector<dxb200_image> ds(src + i, src + k), dd;
+        if (dst) dd.assign(dst + i, dst + k);
         size_t offIn = 0, offOut = 0;
         for (size_t m = i; m < k && hr == DXB_S_OK; ++m)
         {
             ds[m - i].pixels = static_cast<uint8_t*>(t_v.lane->dIn[slot]) + offIn;
-            dd[m - i].pixels = static_cast<uint8_t*>(t_v.lane->dOut[slot]) + offOut;
             hr = cuda_hr(cudaMemcpyAsync(ds[m - i].pixels, src[m].pixels, src[m].slicePitch, cudaMemcpyHostToDevice, st), "H2D");
             offIn += (src[m].slicePitch + 255) & ~size_t(255);
+            if (!dst) continue;
+            dd[m - i].pixels = static_cast<uint8_t*>(t_v.lane->dOut[slot]) + offOut;
+            if (dstIn && hr == DXB_S_OK) hr = cuda_hr(cudaMemcpyAsync(dd[m - i].pixels, dst[m].pixels, dst[m].slicePitch, cudaMemcpyHostToDevice, st), "H2D");
             offOut += (dst[m].slicePitch + 255) & ~size_t(255);
         }
         if (hr) break;
-        hr = fn(ds.data(), dd.data(), k - i, st); if (hr) break;
-        for (size_t m = i; m < k && hr == DXB_S_OK; ++m)
+        hr = fn(ds.data(), dst ? dd.data() : nullptr, k - i, st); if (hr) break;
+        for (size_t m = i; m < k && hr == DXB_S_OK && dst && !dstIn; ++m)
             hr = cuda_hr(cudaMemcpyAsync(dst[m].pixels, dd[m - i].pixels, dst[m].slicePitch, cudaMemcpyDeviceToHost, st), "D2H");
         i = k; slot = (slot + 1) % NSLOT;
     }
@@ -1395,6 +1401,262 @@ int32_t dxb200_resize(const dxb200_image* src, size_t nimages, uint32_t filter, 
     if (hr != DXB_S_OK) return hr;
     return run_sharded(nimages, [&](size_t i) { return src[i].slicePitch + dst[i].slicePitch; },
         [&](size_t lo, size_t hi) { return resize_host_range(src, dst, lo, hi, filter, mode); });
+}
+
+} // extern "C"
+
+// ---- ComputeMSE (DirectXTexMisc.cpp:388-468) and the IsAlphaAllOpaque scan (DirectXTexImage.cpp:800-852) ------------------------
+// dxb_analyze.cuh states the arithmetic and the fixed fp64 reduction tree; here: validation, chunk bookkeeping, staging.
+#include "dxb_analyze.cuh"
+
+namespace {
+
+// IsValid (DirectXTex.inl:57-60); every valid format this backend does not implement (typeless, planar, palettized, video, ...)
+// is HRESULT_E_NOT_SUPPORTED (:395-407: no CPU fallback)
+int32_t check_analyze_format(uint32_t f)
+{
+    if (f < 1u || f > 191u) return DXB_E_INVALIDARG;
+    return (is_compressed(f) || is_supported_pixel_format(f)) ? DXB_S_OK : DXB_E_NOT_SUPPORTED;
+}
+
+uint32_t tile_rows(const dxb200_image& im) { return (uint32_t)((im.height + 3) / 4); }
+uint32_t chunks_per_row(const dxb200_image& im) { return (uint32_t)(((im.width + 3) / 4 + DXB_AN_TILES - 1) / DXB_AN_TILES); }
+
+int32_t plan_mse(const dxb200_image* a, const dxb200_image* b, size_t n)
+{
+    if (!a || !b || !n) return DXB_E_INVALIDARG;
+    uint64_t chunks = 0;
+    for (size_t i = 0; i < n; ++i)
+    {
+        if (!a[i].pixels || !b[i].pixels) return DXB_E_POINTER;
+        if (a[i].width != b[i].width || a[i].height != b[i].height) return DXB_E_INVALIDARG;
+        const int32_t ha = check_analyze_format(a[i].format), hb = check_analyze_format(b[i].format);
+        if (ha == DXB_E_INVALIDARG || hb == DXB_E_INVALIDARG) return DXB_E_INVALIDARG;
+        if (ha != DXB_S_OK || hb != DXB_S_OK) return DXB_E_NOT_SUPPORTED;
+        if (!a[i].width || !a[i].height || a[i].width > 0xFFFFFFFFull || a[i].height > 0xFFFFFFFFull) return DXB_E_INVALIDARG;
+        chunks += (uint64_t)tile_rows(a[i]) * chunks_per_row(a[i]);
+        if (chunks > 0x7FFFFFFFull) return DXB_E_INVALIDARG;
+    }
+    return DXB_S_OK;
+}
+
+// enqueue the chunk kernels for pairs whose pixels live on the device: pair i writes its partials (4 doubles per chunk) from
+// partials + 4 * firstPartial[i] on.  Pairs are grouped by the kind of their sides (BC or not), one launch per kind.
+int32_t launch_mse(const dxb200_image* a, const dxb200_image* b, size_t n, uint32_t flags, const uint32_t* firstPartial, double* partials, cudaStream_t stream)
+{
+    std::vector<dxb_pair_job> kinds[3];
+    for (size_t i = 0; i < n; ++i)
+    {
+        dxb_pair_job j; memset(&j, 0, sizeof(j));
+        const bool bcA = is_compressed(a[i].format), bcB = is_compressed(b[i].format);
+        const bool swap = !bcA && bcB;                           // a lone BC side goes first
+        const dxb200_image& x = swap ? b[i] : a[i];
+        const dxb200_image& y = swap ? a[i] : b[i];
+        uint32_t f = (flags & DXB_CMSE_MASK) | dxb_cmse_implied(a[i].format, false) | dxb_cmse_implied(b[i].format, true);
+        if (swap) f = dxb_cmse_swap(f);
+        j.a = x.pixels; j.b = y.pixels; j.pitchA = x.rowPitch; j.pitchB = y.rowPitch;
+        j.fmtA = x.format; j.fmtB = y.format; j.flags = f;
+        j.width = (uint32_t)x.width; j.height = (uint32_t)x.height;
+        j.nbx = (j.width + 3) / 4; j.cpr = chunks_per_row(x);
+        j.firstPartial = firstPartial[i];
+        kinds[(bcA && bcB) ? 2 : (bcA || bcB) ? 1 : 0].push_back(j);
+    }
+    int32_t hr = DXB_S_OK;
+    for (auto& jobs : kinds)
+    {
+        if (jobs.empty() || hr != DXB_S_OK) continue;
+        uint64_t total = 0;
+        for (auto& j : jobs) { j.firstUnit = (uint32_t)total; total += (uint64_t)((j.height + 3) / 4) * j.cpr; }
+        DeviceJobs<dxb_pair_job> dj;
+        hr = dj.upload(jobs, stream);
+        if (hr != DXB_S_OK) return hr;
+        const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(total, (uint64_t)t_v.dev->gridRow));
+        dxb_launch_compute_mse(grid, stream, dj.d, jobs[0], (uint32_t)jobs.size(), (uint32_t)total, partials);
+        hr = check_launch("k_compute_mse");
+        dj.release();
+    }
+    return hr;
+}
+
+int32_t plan_opaque(const dxb200_image* images, size_t n)
+{
+    if (!images || !n) return DXB_E_INVALIDARG;
+    const uint32_t fmt = images[0].format;
+    for (size_t i = 0; i < n; ++i)
+    {
+        if (!images[i].pixels) return DXB_E_POINTER;
+        if (images[i].format != fmt) return DXB_E_INVALIDARG;
+        if (!images[i].width || !images[i].height || images[i].width > 0xFFFFFFFFull || images[i].height > 0xFFFFFFFFull) return DXB_E_INVALIDARG;
+    }
+    uint64_t chunks = 0;
+    for (size_t i = 0; i < n; ++i) chunks += (uint64_t)tile_rows(images[i]) * chunks_per_row(images[i]);
+    if (chunks > 0x7FFFFFFFull) return DXB_E_INVALIDARG;
+    return check_analyze_format(fmt);
+}
+
+// BC formats without an alpha scan (BC4 / BC5 / BC6H): "not opaque" for every image (IsAlphaAllOpaqueBC :569-572)
+bool opaque_trivially_false(uint32_t fmt) { return is_compressed(fmt) && !dxb_opaque_bc_scanned(fmt); }
+
+// enqueue the scan of device images; *opaque (device) must hold 1 before, is set to 0 by a tile with a pixel below the threshold
+int32_t launch_opaque(const dxb200_image* images, size_t n, int32_t* opaque, cudaStream_t stream)
+{
+    std::vector<dxb_pair_job> jobs(n);
+    uint64_t total = 0;
+    for (size_t i = 0; i < n; ++i)
+    {
+        dxb_pair_job& j = jobs[i]; memset(&j, 0, sizeof(j));
+        j.a = images[i].pixels; j.pitchA = images[i].rowPitch; j.fmtA = images[i].format;
+        j.width = (uint32_t)images[i].width; j.height = (uint32_t)images[i].height;
+        j.nbx = (j.width + 3) / 4; j.cpr = chunks_per_row(images[i]);
+        j.firstUnit = (uint32_t)total; total += (uint64_t)tile_rows(images[i]) * j.cpr;
+    }
+    DeviceJobs<dxb_pair_job> dj;
+    int32_t hr = dj.upload(jobs, stream);
+    if (hr != DXB_S_OK) return hr;
+    const uint32_t grid = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(total, (uint64_t)t_v.dev->gridRow));
+    dxb_launch_alpha_opaque(grid, stream, dj.d, jobs[0], (uint32_t)n, (uint32_t)total, opaque);
+    hr = check_launch("k_alpha_opaque");
+    dj.release();
+    return hr;
+}
+
+} // namespace
+
+extern "C" {
+
+int32_t dxb200_compute_mse_device(const dxb200_image* a, const dxb200_image* b, size_t n, uint32_t flags, float* out, void* stream)
+{
+    int32_t hr = plan_mse(a, b, n);
+    if (hr != DXB_S_OK) return hr;
+    if (!out) return DXB_E_POINTER;
+    DevScope scope;
+    hr = scope.enter(a[0].pixels);
+    if (hr != DXB_S_OK) return hr;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    std::vector<uint32_t> first(n);
+    std::vector<dxb_mse_final> fin(n);
+    uint32_t chunks = 0;
+    for (size_t i = 0; i < n; ++i)
+    {
+        const uint32_t c = tile_rows(a[i]) * chunks_per_row(a[i]);
+        first[i] = chunks;
+        fin[i].pixels = (uint64_t)a[i].width * a[i].height; fin[i].firstPartial = chunks; fin[i].nchunks = c;
+        chunks += c;
+    }
+    double* dPart = nullptr;
+    dxb_mse_final* dFin = nullptr;
+    DXB_CUDA(cudaMallocAsync(reinterpret_cast<void**>(&dPart), (size_t)chunks * 4 * sizeof(double), st));
+    hr = cuda_hr(cudaMallocAsync(reinterpret_cast<void**>(&dFin), n * sizeof(dxb_mse_final), st), "cudaMallocAsync");
+    if (hr == DXB_S_OK) hr = cuda_hr(cudaMemcpyAsync(dFin, fin.data(), n * sizeof(dxb_mse_final), cudaMemcpyHostToDevice, st), "H2D");
+    if (hr == DXB_S_OK) hr = launch_mse(a, b, n, flags, first.data(), dPart, st);
+    if (hr == DXB_S_OK)
+    {
+        dxb_launch_mse_finish(st, dFin, (uint32_t)n, dPart, out);
+        hr = check_launch("k_mse_finish");
+    }
+    cudaFreeAsync(dPart, st);
+    if (dFin) cudaFreeAsync(dFin, st);
+    return hr;
+}
+
+int32_t dxb200_compute_mse(const dxb200_image* a, const dxb200_image* b, size_t n, uint32_t flags, float* mse, float* mseV)
+{
+    int32_t hr = plan_mse(a, b, n);
+    if (hr != DXB_S_OK) return hr;
+    if (!mse) return DXB_E_POINTER;
+    // bands of whole tile rows (4 pixel rows, 1 block row); their chunk partials land where a whole-image launch puts them
+    std::vector<dxb200_image> ba, bb;
+    std::vector<size_t> bandImage;
+    for (size_t i = 0; i < n; ++i)
+    {
+        BandSplit s;
+        split_bands(a + i, b + i, 1, is_compressed(a[i].format) ? 1 : 4, is_compressed(b[i].format) ? 1 : 4, is_compressed(a[i].format), is_compressed(b[i].format), s);
+        ba.insert(ba.end(), s.src.begin(), s.src.end()); bb.insert(bb.end(), s.dst.begin(), s.dst.end());
+        bandImage.insert(bandImage.end(), s.src.size(), i);
+    }
+    std::vector<uint32_t> first(ba.size() + 1, 0);
+    for (size_t k = 0; k < ba.size(); ++k) first[k + 1] = first[k] + tile_rows(ba[k]) * chunks_per_row(ba[k]);
+    std::vector<double> partials((size_t)first.back() * 4);
+    hr = run_sharded(ba.size(), [&](size_t k) { return ba[k].slicePitch + bb[k].slicePitch; },
+        [&](size_t lo, size_t hi) -> int32_t
+        {
+            const size_t count = (size_t)(first[hi] - first[lo]) * 4;
+            double* dPart = nullptr;
+            DXB_CUDA(cudaMalloc(reinterpret_cast<void**>(&dPart), std::max<size_t>(count, 1) * sizeof(double)));
+            size_t next = lo;
+            int32_t h2 = run_staged(ba.data() + lo, bb.data() + lo, hi - lo,
+                [&](const dxb200_image* da, const dxb200_image* db, size_t cnt, cudaStream_t st)
+                {
+                    std::vector<uint32_t> fp(cnt);
+                    for (size_t m = 0; m < cnt; ++m) fp[m] = first[next + m] - first[lo];
+                    next += cnt;
+                    return launch_mse(da, db, cnt, flags, fp.data(), dPart, st);
+                }, nullptr, nullptr, true);
+            if (h2 == DXB_S_OK) h2 = cuda_hr(cudaMemcpy(partials.data() + (size_t)first[lo] * 4, dPart, count * sizeof(double), cudaMemcpyDeviceToHost), "D2H partials");
+            cudaFree(dPart);
+            return h2;
+        });
+    if (hr != DXB_S_OK) return hr;
+    // the image level of the tree, on the host (the same IEEE fp64 additions as k_mse_finish)
+    size_t k = 0;
+    for (size_t i = 0; i < n; ++i)
+    {
+        const uint32_t p0 = first[k];
+        while (k < ba.size() && bandImage[k] == i) ++k;
+        float o[5];
+        dxb_cmse_finish(partials.data() + (size_t)p0 * 4, first[k] - p0, (uint64_t)a[i].width * a[i].height, o);
+        mse[i] = o[0];
+        if (mseV) memcpy(mseV + 4 * i, o + 1, 4 * sizeof(float));
+    }
+    return DXB_S_OK;
+}
+
+int32_t dxb200_is_alpha_all_opaque_device(const dxb200_image* images, size_t n, int32_t* opaque, void* stream)
+{
+    int32_t hr = plan_opaque(images, n);
+    if (hr != DXB_S_OK) return hr;
+    if (!opaque) return DXB_E_POINTER;
+    DevScope scope;
+    hr = scope.enter(images[0].pixels);
+    if (hr != DXB_S_OK) return hr;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const bool none = opaque_trivially_false(images[0].format);
+    dxb_launch_set_i32(st, opaque, none ? 0 : 1);
+    hr = check_launch("k_set_i32");
+    if (hr == DXB_S_OK && !none) hr = launch_opaque(images, n, opaque, st);
+    return hr;
+}
+
+int32_t dxb200_is_alpha_all_opaque(const dxb200_image* images, size_t n, int32_t* opaque)
+{
+    int32_t hr = plan_opaque(images, n);
+    if (hr != DXB_S_OK) return hr;
+    if (!opaque) return DXB_E_POINTER;
+    if (opaque_trivially_false(images[0].format)) { *opaque = 0; return DXB_S_OK; }
+    const bool bc = is_compressed(images[0].format);
+    BandSplit bands;
+    split_bands(images, images, n, bc ? 1 : 4, bc ? 1 : 4, bc, bc, bands);
+    std::atomic<int32_t> result{1};
+    hr = run_sharded(bands.src.size(), [&](size_t k) { return bands.src[k].slicePitch; },
+        [&](size_t lo, size_t hi) -> int32_t
+        {
+            int32_t* dFlag = nullptr;
+            DXB_CUDA(cudaMalloc(reinterpret_cast<void**>(&dFlag), sizeof(int32_t)));
+            int32_t h2 = DXB_S_OK, found = 1;
+            dxb_launch_set_i32(t_v.lane->streams[0], dFlag, 1);
+            h2 = check_launch("k_set_i32");
+            if (h2 == DXB_S_OK) h2 = cuda_hr(cudaStreamSynchronize(t_v.lane->streams[0]), "flag init");
+            if (h2 == DXB_S_OK)
+                h2 = run_staged(bands.src.data() + lo, nullptr, hi - lo,
+                    [&](const dxb200_image* ds, const dxb200_image*, size_t cnt, cudaStream_t st) { return launch_opaque(ds, cnt, dFlag, st); });
+            if (h2 == DXB_S_OK) h2 = cuda_hr(cudaMemcpy(&found, dFlag, sizeof(int32_t), cudaMemcpyDeviceToHost), "D2H flag");
+            if (h2 == DXB_S_OK && found == 0) result.store(0);
+            cudaFree(dFlag);
+            return h2;
+        });
+    if (hr != DXB_S_OK) return hr;
+    *opaque = result.load();
+    return DXB_S_OK;
 }
 
 } // extern "C"

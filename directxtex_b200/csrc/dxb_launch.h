@@ -16,6 +16,27 @@ struct dxb_job
     uint32_t pad;
 };
 
+// one image pair (ComputeMSE: a vs b) or one image (IsAlphaAllOpaque: a) walked one thread per 4x4 tile; the work units are
+// chunks of DXB_AN_TILES tiles of one tile row (dxb_analyze.cuh), cpr per tile row
+struct dxb_pair_job
+{
+    const uint8_t* a; const uint8_t* b;
+    size_t pitchA, pitchB;
+    uint32_t width, height;
+    uint32_t fmtA, fmtB;
+    uint32_t flags;                // CMSE flags, the ones implied by the formats included
+    uint32_t nbx, cpr;             // tiles per row, chunks per tile row
+    uint32_t firstUnit;            // first chunk of this job in the launch
+    uint32_t firstPartial;         // index of its first chunk partial (ComputeMSE)
+    uint32_t pad;
+};
+// image level of ComputeMSE: chunks [firstPartial, firstPartial + nchunks) of the partials -> out[5 * index ..]
+struct dxb_mse_final
+{
+    uint64_t pixels;
+    uint32_t firstPartial, nchunks;
+};
+
 struct dxb_compress_params
 {
     uint32_t srcFormat, dstFormat;
@@ -73,6 +94,14 @@ void dxb_launch_scale_alpha(unsigned grid, cudaStream_t stream, const dxb_job& j
 void dxb_launch_pmalpha(unsigned grid, cudaStream_t stream, const dxb_job* jobs, const dxb_job* hostJobs, const dxb_convert_params& P);
 bool dxb_launch_mip_box3(cudaStream_t stream, const dxb_mip_job* jobsDev, const dxb_mip_job* hostJobs, uint32_t items, const dxb_mip_params& P);
 bool dxb_launch_mip_tail(cudaStream_t stream, const dxb_mip_job* jobsDev, uint32_t items, uint32_t count, const dxb_mip_params& P);
+// ComputeMSE / IsAlphaAllOpaque (dxb_k_analyze.cu); every job of one launch has the same kind of sides (BC or not, BC on side a
+// when only one is); partials = 4 doubles per chunk
+void dxb_launch_compute_mse(unsigned grid, cudaStream_t stream, const dxb_pair_job* jobs, const dxb_pair_job& single, uint32_t njobs,
+                            uint32_t totalUnits, double* partials);
+void dxb_launch_mse_finish(cudaStream_t stream, const dxb_mse_final* jobs, uint32_t njobs, const double* partials, float* out);
+void dxb_launch_alpha_opaque(unsigned grid, cudaStream_t stream, const dxb_pair_job* jobs, const dxb_pair_job& single, uint32_t njobs,
+                             uint32_t totalUnits, int32_t* opaque);
+void dxb_launch_set_i32(cudaStream_t stream, int32_t* p, int32_t value);
 // resident CTAs per SM of each kernel at its block size
 int dxb_occupancy_bc15();
 int dxb_occupancy_bc7();

@@ -571,6 +571,34 @@ HRESULT CompressEx(const Image* srcImages, size_t nimages, const TexMetadata& me
 }
 
 // ---------------------------------------------------------------------------------------------------
+// ComputeMSE (DirectXTexMisc.cpp:388-468) and ScratchImage::IsAlphaAllOpaque (DirectXTexImage.cpp:800-852)
+HRESULT ComputeMSE(const Image& image1, const Image& image2, float& mse, float* mseV, CMSE_FLAGS flags) noexcept
+{
+    const dxb200_image a = to_c(image1), b = to_c(image2);
+    return dxb200_compute_mse(&a, &b, 1, static_cast<uint32_t>(flags), &mse, mseV);
+}
+
+bool ScratchImage::IsAlphaAllOpaque() const noexcept
+{
+    if (!m_image) return false;
+    if (!HasAlpha(m_metadata.format)) return true;
+    DXGI_FORMAT f = m_metadata.format;
+    switch (f)                     // IsAlphaAllOpaqueBC promotes the typeless BC formats (DirectXTexCompress.cpp:545-553)
+    {
+    case DXGI_FORMAT_BC1_TYPELESS: f = DXGI_FORMAT_BC1_UNORM; break;
+    case DXGI_FORMAT_BC2_TYPELESS: f = DXGI_FORMAT_BC2_UNORM; break;
+    case DXGI_FORMAT_BC3_TYPELESS: f = DXGI_FORMAT_BC3_UNORM; break;
+    case DXGI_FORMAT_BC7_TYPELESS: f = DXGI_FORMAT_BC7_UNORM; break;
+    default: break;
+    }
+    std::vector<dxb200_image> imgs(m_nimages);
+    for (size_t i = 0; i < m_nimages; ++i) { imgs[i] = to_c(m_image[i]); imgs[i].format = static_cast<uint32_t>(f); }
+    int32_t opaque = 0;
+    if (FAILED(dxb200_is_alpha_all_opaque(imgs.data(), imgs.size(), &opaque))) return false;
+    return opaque != 0;
+}
+
+// ---------------------------------------------------------------------------------------------------
 // Decompress
 HRESULT Decompress(const Image& cImage, DXGI_FORMAT format, ScratchImage& image) noexcept
 {

@@ -8,6 +8,7 @@
 // Provided besides the accelerated operations: the containers (ScratchImage / Image / TexMetadata / Blob with every constructor of the 2D
 // path), every DXGI format utility, ComputePitch with all CP_FLAGS, the DDS container.  Not provided (out of the hot path, SURVEY.md 8):
 // WIC / TGA / HDR / EXR codecs, D3D interop, 3D textures, normal maps, TransformImage / EvaluateImage / CopyRectangle / FlipRotate.
+// ComputeMSE and ScratchImage::IsAlphaAllOpaque run on the device (BC data decoded in the kernel).
 #pragma once
 #include <cstddef>
 #include <cstdint>
@@ -180,6 +181,9 @@ namespace DirectX
         size_t GetImageCount() const noexcept { return m_nimages; }
         uint8_t* GetPixels() const noexcept { return m_memory; }
         size_t GetPixelsSize() const noexcept { return m_size; }
+        // DirectXTexImage.cpp:800-852: false without images, true for formats without alpha, else the scan of every image on the
+        // device (dxb200_is_alpha_all_opaque); false on any failure, the reference's failure value
+        bool IsAlphaAllOpaque() const noexcept;
 
     private:
         size_t m_nimages, m_size;
@@ -251,6 +255,18 @@ namespace DirectX
     DXTEXB200_API HRESULT Compress(const Image* srcImages, size_t nimages, const TexMetadata& metadata, DXGI_FORMAT format, TEX_COMPRESS_FLAGS compress, float threshold, ScratchImage& cImages) noexcept;
     DXTEXB200_API HRESULT CompressEx(const Image& srcImage, DXGI_FORMAT format, const CompressOptions& options, ScratchImage& cImage, std::function<bool(size_t, size_t)> statusCallBack = nullptr);
     DXTEXB200_API HRESULT CompressEx(const Image* srcImages, size_t nimages, const TexMetadata& metadata, DXGI_FORMAT format, const CompressOptions& options, ScratchImage& cImages, std::function<bool(size_t, size_t)> statusCallBack = nullptr);
+
+    // DirectXTex.h:1022-1041 (ComputeMSE): mseV within 4 fp32 ulp of the exact mean of the reference's per-pixel squares, see
+    // include/dxtex_b200.h (dxb200_compute_mse)
+    enum CMSE_FLAGS : uint32_t
+    {
+        CMSE_DEFAULT = 0,
+        CMSE_IMAGE1_SRGB = 0x1, CMSE_IMAGE2_SRGB = 0x2,
+        CMSE_IGNORE_RED = 0x10, CMSE_IGNORE_GREEN = 0x20, CMSE_IGNORE_BLUE = 0x40, CMSE_IGNORE_ALPHA = 0x80,
+        CMSE_IMAGE1_X2_BIAS = 0x100, CMSE_IMAGE2_X2_BIAS = 0x200,
+    };
+    constexpr CMSE_FLAGS operator|(CMSE_FLAGS a, CMSE_FLAGS b) noexcept { return static_cast<CMSE_FLAGS>(static_cast<uint32_t>(a) | static_cast<uint32_t>(b)); }
+    DXTEXB200_API HRESULT ComputeMSE(const Image& image1, const Image& image2, float& mse, float* mseV, CMSE_FLAGS flags = CMSE_DEFAULT) noexcept;
 
     DXTEXB200_API HRESULT Decompress(const Image& cImage, DXGI_FORMAT format, ScratchImage& image) noexcept;
     DXTEXB200_API HRESULT Decompress(const Image* cImages, size_t nimages, const TexMetadata& metadata, DXGI_FORMAT format, ScratchImage& images) noexcept;

@@ -1,5 +1,5 @@
 /* dxtex_b200.h — C ABI of libdxtex_b200.so, the B200 (sm_100a) backend for the DirectXTex hot path:
- * DirectX::Compress / Decompress-side block codecs, DirectX::Convert, DirectX::GenerateMipMaps.
+ * DirectX::Compress / Decompress-side block codecs, DirectX::Convert, DirectX::GenerateMipMaps, DirectX::ComputeMSE.
  *
  * Every entry point names the reference interface it replaces (paths relative to the reference
  * repository microsoft/DirectXTex @ 0bb96f0).  The design precedent inside the reference for an
@@ -151,6 +151,26 @@ DXB200_API int32_t  dxb200_premultiply_alpha_device(const dxb200_image* src, siz
 DXB200_API int32_t  dxb200_scale_mipmaps_alpha_for_coverage(const dxb200_image* src, size_t nlevels, float alphaReference, const dxb200_image* dst);
 DXB200_API int32_t  dxb200_scale_mipmaps_alpha_for_coverage_device(const dxb200_image* src, size_t nlevels, float alphaReference,
                                                                    const dxb200_image* dst, void* stream);
+
+/* DirectX::ComputeMSE (DirectXTexMisc.cpp:388-468) for n pairs a[i] vs b[i] (same width / height per pair; any implemented format on
+ * either side, BC included: BC data is decoded in the kernel exactly as Decompress(..., R32G32B32A32_FLOAT) would).
+ *   flags = CMSE_FLAGS (DirectXTex.h:1022-1038); the flags implied by the formats (:46-91) are added per pair.
+ *   mse[i] and mseV[4 * i .. 4 * i + 3] (mseV may be NULL) as the reference returns them.
+ * Per-pixel squares are the reference's fp32 values (up to a few ulp of powf with the sRGB flags); they are summed in fp64 over a
+ * reduction tree fixed by the image geometry (dxb_analyze.cuh), so mseV is within 4 fp32 ulp of the exact mean of those squares
+ * and bit-identical across calls, batch compositions, device counts and the host / device variants.  The reference's running
+ * fp32 sum drifts from the exact value as images grow (~1e-3 relative at 1024^2).
+ * Errors: NULL pixels -> E_POINTER; size mismatch or invalid format -> E_INVALIDARG; typeless / planar / palettized or any
+ * other valid format this backend does not implement -> HRESULT_E_NOT_SUPPORTED; no device -> E_FAIL.
+ * _device: device images, out = 5 floats per pair on the device (mse, then mseV); only enqueues work on `stream`. */
+DXB200_API int32_t  dxb200_compute_mse(const dxb200_image* a, const dxb200_image* b, size_t n, uint32_t flags, float* mse, float* mseV);
+DXB200_API int32_t  dxb200_compute_mse_device(const dxb200_image* a, const dxb200_image* b, size_t n, uint32_t flags, float* out, void* stream);
+/* The image scan of ScratchImage::IsAlphaAllOpaque (DirectXTexImage.cpp:800-852; IsAlphaAllOpaqueBC, DirectXTexCompress.cpp:539-620) over
+ * n images of one format: *opaque = 1 when no in-image pixel has alpha < 0.997 (uncompressed, after load) or < 0.99 (BC1/2/3/7, after
+ * decode), else 0; BC4 / BC5 / BC6H give 0 as IsAlphaAllOpaqueBC does (the HasAlpha test of the ScratchImage member comes first in
+ * the C++ mirror).  Errors as dxb200_compute_mse.  _device: device images and a device int32; only enqueues work. */
+DXB200_API int32_t  dxb200_is_alpha_all_opaque(const dxb200_image* images, size_t n, int32_t* opaque);
+DXB200_API int32_t  dxb200_is_alpha_all_opaque_device(const dxb200_image* images, size_t n, int32_t* opaque, void* stream);
 
 /* ---- DDS container (host-side only, no GPU work; SURVEY 8(f) rank 3) ------------------------------------------------
  * dxb200_metadata is a field-for-field mirror of DirectX::TexMetadata (DirectXTex.h:187-216).
